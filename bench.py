@@ -5,7 +5,7 @@ A "step" is one pass of the hot path over one batch: `batch` published events fa
 every GPU's shard (one fan-out kernel launch per GPU).  Headline unit (BASELINE.md §3): deliveries/s = 32-byte records
 landed in mailboxes per second, whole job; publishes/s is reported beside it.
 
-  python bench.py [--gpus N --steps K --warmup W] [--workload default|config2|config3|config5]
+  python bench.py [--gpus N --steps K --warmup W] [--workload default|config2|config3|config5] [--dump-outputs DIR]
   python bench.py --impl reference ...      # the reference's CPU path (restated Go bus) on the host cores
 
 Default: the headline is BASELINE config 3 — the configuration north_star's target is quoted on (1,048,576 subscribers
@@ -64,6 +64,8 @@ def parse():
     ap.add_argument("--no-extras", action="store_true", help="default workload: headline only")
     ap.add_argument("--no-verify", action="store_true", help="skip the in-bench oracle check (diagnostics only; the line says so)")
     ap.add_argument("--max-steps", type=int, default=40_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what each configuration's timed fan-out left in the "
+                    "mailboxes after its last step to DIR/<config>_<array>.npy (float64, a seeded sample; see dump_outputs)")
     return ap.parse_args()
 
 
@@ -304,16 +306,12 @@ def run_config(cx, name: str, headline: bool):
     sampler = ClockSampler(local)
     sampler.start()                                            # started early so NVML is warm before the timed region
     run_steps(warmup)
-    # settle: a fresh box pages in driver/library code lazily; keep warming (untimed) for ~0.3 s of wall clock
-    settle, t_settle = 0, time.perf_counter()
-    settle_chunk = 100 if n_subs <= 131_072 else 10
-    while settle < 20_000:
-        run_steps(settle_chunk); torch.cuda.synchronize(); settle += settle_chunk
-        done = time.perf_counter() - t_settle >= 0.3
-        if world > 1:                                          # every rank issues the same number of steps: rank 0's clock decides
-            t_ = torch.tensor([1 if done else 0], device=dev); dist.broadcast(t_, src=0); done = bool(int(t_.item()))
-        if done:
-            break
+    # settle: a fresh box pages in driver/library code lazily; keep warming (untimed) for 1.2e11 records' worth of
+    # all-ones fan-out, about 0.6 s on a B200.  A step count rather than a clock, so that every run (and every build)
+    # times the same batches of the same trace and leaves the same mailbox contents behind.
+    settle = int(min(20_000, max(10, round(1.2e11 / (n_subs * B)))))
+    run_steps(settle)
+    torch.cuda.synchronize()
     # if the timed region would straddle the end of the trace, start it at the next cycle instead (re-stamp outside the timing)
     pos = state["step"] % n_trace_batches
     if steps <= n_trace_batches and pos + steps > n_trace_batches:
@@ -340,6 +338,8 @@ def run_config(cx, name: str, headline: bool):
         dist.all_reduce(deliv, op=dist.ReduceOp.SUM)
     deliveries, ticks = float(deliv[0].item()), float(deliv[1].item())
     launches = st1["kernel_launches"] - st0["kernel_launches"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, name, bus, first, n_subs, R)
     value = deliveries / (ms * 1e-3)
     publishes_per_s = steps * B / (ms * 1e-3)
 
@@ -557,6 +557,34 @@ def run_lossless_and_bridge(cx):
               "value": total / med, "unit": "records/s", "gb_per_s": total * 32 / med / 1e9, "ms_per_call": med * 1e3, "records_per_call": total}
     bus.close()
     return lossless, bridge
+
+
+DUMP_SUBS, DUMP_WINDOWS = 65_536, 64
+
+
+def _words(a) -> np.ndarray:
+    """Unsigned integers as float64, 64-bit ones split into their two 32-bit halves (low first): exact at any value."""
+    return np.ascontiguousarray(a).view(np.uint32).astype(np.float64)
+
+
+def dump_outputs(out_dir, name, bus, first, n_subs, ring_cap):
+    """What a caller reads back after the timed fan-out's last step, for this rank's shard: delivered count and digest of
+    a seeded sample of subscribers, the mailbox windows (what cpbus_peek_window returns) of a smaller sample, and the
+    shard's digest fold.  The sample depends only on the subscriber count; a configuration writes at most 7 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0xC0DEB2D0)
+    subs = np.sort(rng.choice(n_subs, min(n_subs, DUMP_SUBS), replace=False))
+    dg = bus.digests(first, n_subs)[subs]
+    win_subs = np.sort(rng.choice(subs, min(len(subs), DUMP_WINDOWS), replace=False))
+    windows = np.full((len(win_subs), ring_cap, 8), -1.0)     # 8 words per record; rows of -1 past a short window
+    for k, s in enumerate(win_subs):
+        w = _words(bus.peek_window(first + int(s))).reshape(-1, 8)
+        windows[k, :len(w)] = w
+    arrays = {"subscribers": (first + subs).astype(np.float64), "count": _words(dg["count"]).reshape(-1, 2),
+              "digest": _words(dg["digest"]).reshape(-1, 2), "window_subscribers": (first + win_subs).astype(np.float64),
+              "windows": windows, "fold": _words(np.array(bus.digest_fold(first, n_subs), dtype=np.uint64)).reshape(4, 2)}
+    for key, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}_{key}.npy"), a)
 
 
 def verify(cx, name, sb, log, base, masks, n_subs, B, K_timers, timer_src0, slot_hist, make_records):
