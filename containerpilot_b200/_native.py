@@ -64,6 +64,8 @@ _P = C.POINTER
 SYMBOLS = {
     "cpbus_create": (C.c_int, [_P(Config), _P(C.c_void_p)]),
     "cpbus_destroy": (C.c_int, [C.c_void_p]),
+    "cpbus_create_sharded": (C.c_int, [_P(Config), _P(C.c_int32), C.c_uint32, _P(C.c_void_p)]),
+    "cpbus_shard_range": (C.c_int, [C.c_uint32, C.c_uint32, C.c_uint32, _P(C.c_uint32), _P(C.c_uint32)]),
     "cpbus_intern": (C.c_int, [C.c_void_p, C.c_char_p, C.c_size_t, _P(C.c_uint32)]),
     "cpbus_source": (C.c_int, [C.c_void_p, C.c_uint32, C.c_char_p, C.c_size_t, _P(C.c_size_t)]),
     "cpbus_intern_ephemeral": (C.c_int, [C.c_void_p, C.c_char_p, C.c_size_t, _P(C.c_uint32)]),

@@ -19,7 +19,10 @@ assert EVENT_DTYPE.itemsize == 32
 class Bus:
     def __init__(self, n_max_subs: int, ring_cap: int = 1024, batch_cap: int = 256, timers_per_sub: int = 0,
                  lossless: bool = False, digest: bool = True, device: int = -1, sub_id_base: int = 0,
-                 store_path: int = nat.STORE_AUTO, stream: int | None = None, grid_ctas: int = 0):
+                 store_path: int = nat.STORE_AUTO, stream: int | None = None, grid_ctas: int = 0, devices=None):
+        """`devices`: a list of CUDA ordinals makes this ONE handle over len(devices) shards (`cpbus_create_sharded`):
+        shard k on devices[k], the same ids, records and digests as one bus with the same arguments; `device` is then
+        ignored."""
         self._lib = nat.load()
         cfg = nat.Config()
         cfg.n_max_subs, cfg.ring_cap, cfg.batch_cap, cfg.timers_per_sub = n_max_subs, ring_cap, batch_cap, timers_per_sub
@@ -27,7 +30,11 @@ class Bus:
         cfg.device, cfg.sub_id_base, cfg.store_path, cfg.grid_ctas = device, sub_id_base, store_path, grid_ctas
         cfg.stream = C.c_void_p(stream) if stream else None
         self._h = C.c_void_p()
-        nat.check(self._lib.cpbus_create(C.byref(cfg), C.byref(self._h)), "cpbus_create")
+        if devices is None:
+            nat.check(self._lib.cpbus_create(C.byref(cfg), C.byref(self._h)), "cpbus_create")
+        else:
+            devs = (C.c_int32 * max(1, len(devices)))(*devices)
+            nat.check(self._lib.cpbus_create_sharded(C.byref(cfg), devs, len(devices), C.byref(self._h)), "cpbus_create_sharded")
         self.ring_cap, self.batch_cap, self.sub_id_base = ring_cap, batch_cap, sub_id_base
 
     # -- lifecycle ---------------------------------------------------------

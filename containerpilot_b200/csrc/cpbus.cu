@@ -186,6 +186,18 @@ struct cpbus {
 
   cpbus_stats_t st{};
   std::mutex mu;   // drain/stats from a second thread
+
+  // Sharded handle (cpbus_create_sharded): G shard buses behind this one.  The handle keeps what the kernels never see
+  // (intern table, clock, publish ordinal, debug ring, host publish counts, lossless room bound) and stages events into
+  // h_batch[0]; a flush puts the staged records into the stream owned by shard 0 and fans them out on every shard.
+  std::vector<cpbus*> shards;             // empty: an ordinary bus
+  std::vector<uint32_t> shard_first;      // shard k holds local ids [shard_first[k], shard_first[k+1]) (global = sub_id_base + local)
+  std::vector<cpbus_stream*> shard_st;    // shard k's end of the handle's stream (shard 0 owns it)
+  cpbus_event* d_batch_host = nullptr;    // device alias of the pinned, portable staging buffer (admission reads it in place)
+  bool any_timer = false;                 // a timer has been armed on some shard (cpbus_timer_cancel's "no timer table yet")
+  std::vector<std::pair<uint32_t, uint32_t>> fold_parts[kFoldSlots];   // handle ticket -> (shard, shard ticket)
+  std::vector<uint32_t> result_parts[8];
+  bool sharded() const { return !shards.empty(); }
 };
 
 namespace {
@@ -403,27 +415,39 @@ int launch_fanout(cpbus* b, const cpbus_event* d_src, uint32_t n, uint64_t w, in
   return CPBUS_OK;
 }
 
-// lossless admission (reference: the sender blocks on a full channel, events/subscriber.go:30-32)
-int admit(cpbus* b, const cpbus_event* d_src, uint32_t n, uint64_t w, bool* ok, uint32_t* prefix = nullptr) {
-  *ok = true;
-  if (prefix) *prefix = n;
-  if (!b->lossless || b->n_next == 0) return CPBUS_OK;
-  // the most this launch can append to ONE mailbox: every event of the batch + every firing of its timer slots in the window
+// the most a launch of n events up to watermark w can append to ONE mailbox: every event + every firing of its timer slots
+uint64_t admit_need(uint32_t n, uint32_t K, bool timers, uint64_t min_period, uint64_t last_watermark, uint64_t w) {
   uint64_t need = n;
-  if (b->n_timers && b->K) {
-    const uint64_t per_slot = (b->min_period != UINT64_MAX && w > b->last_watermark) ? (w - b->last_watermark) / b->min_period + 2 : 2;
-    need += (uint64_t)b->K * per_slot;
+  if (timers && K) {
+    const uint64_t per_slot = (min_period != UINT64_MAX && w > last_watermark) ? (w - last_watermark) / min_period + 2 : 2;
+    need += (uint64_t)K * per_slot;
   }
-  if (b->room_lb >= need) { b->room_lb -= need; b->st.admit_skipped++; return CPBUS_OK; }   // provably fits: no kernel, no sync
+  return need;
+}
+
+// enqueue the admission kernel and the D2H of its result words into h_stats (the caller synchronises b->stream)
+int admit_launch(cpbus* b, const cpbus_event* d_src, uint32_t n, uint64_t w) {
   CK(cudaMemsetAsync(&b->d_stats->admit_overflow, 0, 4 * sizeof(unsigned long long), b->stream));   // overflow, overwritten, max_used, deficit
   const uint32_t threads = 256, grid = (b->n_next + threads - 1) / threads;
   admit_kernel<<<grid, threads, 0, b->stream>>>(d_src, n, w, b->d_ctl, b->d_timers, b->n_next, b->R, b->K,
                                                 b->cfg.sub_id_base, b->n_timers > 0 && b->K > 0, b->d_stats,
                                                 b->n_paired > 0 ? b->d_pairs : nullptr);
   CK(cudaGetLastError());
-  b->st.kernel_launches++; b->st.admit_passes++;
+  b->st.kernel_launches++;
   CK(cudaMemcpyAsync(&b->h_stats->admit_overflow, &b->d_stats->admit_overflow, 4 * sizeof(unsigned long long),
                      cudaMemcpyDeviceToHost, b->stream));
+  return CPBUS_OK;
+}
+
+// lossless admission (reference: the sender blocks on a full channel, events/subscriber.go:30-32)
+int admit(cpbus* b, const cpbus_event* d_src, uint32_t n, uint64_t w, bool* ok, uint32_t* prefix = nullptr) {
+  *ok = true;
+  if (prefix) *prefix = n;
+  if (!b->lossless || b->n_next == 0) return CPBUS_OK;
+  const uint64_t need = admit_need(n, b->K, b->n_timers > 0, b->min_period, b->last_watermark, w);
+  if (b->room_lb >= need) { b->room_lb -= need; b->st.admit_skipped++; return CPBUS_OK; }   // provably fits: no kernel, no sync
+  int rc = admit_launch(b, d_src, n, w); if (rc) return rc;
+  b->st.admit_passes++;
   CK(cudaStreamSynchronize(b->stream));
   *ok = b->h_stats->admit_overflow == 0;
   if (!*ok && prefix) *prefix = n - (uint32_t)std::min<unsigned long long>(n, b->h_stats->admit_deficit);   // events every mailbox can still take
@@ -447,7 +471,10 @@ void retire_oneshots(cpbus* b, uint64_t w) {
   if (b->n_timers == 0) b->min_period = UINT64_MAX;
 }
 
+int flush_sharded(cpbus* h, uint64_t w);
+
 int flush_staged(cpbus* b, uint64_t w) {
+  if (b->sharded()) return flush_sharded(b, w);
   const uint32_t n = (uint32_t)b->n_staged;
   if (n == 0 && b->n_timers == 0) { b->last_watermark = std::max(b->last_watermark, w); return CPBUS_OK; }   // nothing armed: the watermark follows the clock
   if (n == 0 && w == b->last_watermark) return CPBUS_OK;
@@ -514,8 +541,17 @@ int flush_staged(cpbus* b, uint64_t w) {
   return CPBUS_OK;
 }
 
+// armed timers; on a sharded handle the sum over its shards
+uint32_t timers_armed(const cpbus* b) {
+  uint32_t n = b->n_timers;
+  for (const cpbus* s : b->shards) n += s->n_timers;
+  return n;
+}
+
+// (a sharded handle keeps min_period the way one bus would; each shard's own bound is never below it, so every shard
+// accepts the handle's step)
 uint64_t max_window(const cpbus* b) {
-  if (!b->K || b->n_timers == 0 || b->min_period == UINT64_MAX) return UINT64_MAX;
+  if (!b->K || timers_armed(b) == 0 || b->min_period == UINT64_MAX) return UINT64_MAX;
   const uint64_t J = 32u / b->K;
   return b->min_period > UINT64_MAX / J ? UINT64_MAX : b->min_period * J;
 }
@@ -528,6 +564,27 @@ int stage_one(cpbus* b, uint32_t code, uint32_t source_id, uint32_t target, uint
 }
 
 bool is_pow2(uint32_t x) { return x && !(x & (x - 1)); }
+
+// ---- sharded handle (cpbus_create_sharded): the entry points below route here; definitions at the end of the file ----
+int sh_subscribe_many(cpbus* h, const uint32_t* masks, uint32_t n, uint32_t* first_sub_id);
+int sh_subscribe_pairs(cpbus* h, uint32_t mask, const cpbus_pair* pairs, uint32_t n_pairs, uint32_t* sub_id);
+int sh_subscribe_pairs_many(cpbus* h, const uint32_t* masks, const cpbus_pair* pairs, const uint32_t* n_pairs, uint32_t n, uint32_t* first_sub_id);
+int sh_unsubscribe(cpbus* h, uint32_t sub_id);
+int sh_set_mask(cpbus* h, uint32_t sub_id, uint32_t mask);
+int sh_timer_add(cpbus* h, uint32_t sub_id, uint64_t period_ns, uint32_t source_id, int oneshot, uint32_t* timer_id);
+int sh_timer_add_many(cpbus* h, uint32_t first_sub, uint32_t n, uint64_t period_ns, const uint32_t* source_ids, uint32_t source_id0, int oneshot);
+int sh_timer_cancel(cpbus* h, uint32_t timer_id);
+int sh_send(cpbus* h, uint32_t sub_id, const cpbus_event* ev);
+int sh_publish_device(cpbus* h, const void* d_events, size_t n, uint64_t watermark_ns);
+int sh_drain_many(cpbus* h, uint32_t first_sub, uint32_t n, cpbus_event* out, size_t cap, uint32_t* offsets, uint32_t* counts, size_t* total);
+int sh_digest(cpbus* h, uint32_t first_sub, uint32_t n, cpbus_digest_t* out);
+int sh_digest_fold_begin(cpbus* h, uint32_t first_sub, uint32_t n, uint32_t* ticket);
+int sh_digest_fold_end(cpbus* h, uint32_t ticket, uint64_t out[4]);
+int sh_step_result_begin(cpbus* h, uint32_t* ticket);
+int sh_step_result_end(cpbus* h, uint32_t ticket, uint64_t out[4]);
+int sh_stats(cpbus* h, cpbus_stats_t* out);
+// the shard that holds the subscriber with global id sub_id, or nullptr (CPBUS_ENOENT) if the handle has not handed it out
+cpbus* sh_owner(const cpbus* h, uint32_t sub_id);
 
 }  // namespace
 
@@ -607,16 +664,23 @@ uint64_t cpbus_record_hash(const cpbus_event* e) {
 }
 uint64_t cpbus_digest_multiplier(void) { return kDigestP; }
 
-int cpbus_create(const cpbus_config* cfg, cpbus_t** out) try {
-  if (!cfg || !out) return CPBUS_EINVAL;
-  *out = nullptr;
+static bool config_ok(const cpbus_config* cfg) {
   const uint32_t R = cfg->ring_cap ? cfg->ring_cap : 1024;
   const uint32_t B = cfg->batch_cap ? cfg->batch_cap : std::min(256u, R / 2);
   const uint32_t K = cfg->timers_per_sub;
-  if (!cfg->n_max_subs || !is_pow2(R) || R < 64 || B == 0 || B > R / 2 || (B % 32) != 0 || B > 1024) return CPBUS_EINVAL;   // 1024: the kernel keeps one match word per 32-event chunk in a lane
-  if (!(K == 0 || K == 1 || K == 2 || K == 4 || K == 8)) return CPBUS_EINVAL;
-  if ((uint64_t)cfg->n_max_subs * std::max(K, 1u) > kTimerSlotMask) return CPBUS_EINVAL;   // timer ids keep 6 generation bits
-  if (cfg->store_path > CPBUS_STORE_BULK) return CPBUS_EINVAL;
+  if (!cfg->n_max_subs || !is_pow2(R) || R < 64 || B == 0 || B > R / 2 || (B % 32) != 0 || B > 1024) return false;   // 1024: the kernel keeps one match word per 32-event chunk in a lane
+  if (!(K == 0 || K == 1 || K == 2 || K == 4 || K == 8)) return false;
+  if ((uint64_t)cfg->n_max_subs * std::max(K, 1u) > kTimerSlotMask) return false;   // timer ids keep 6 generation bits
+  return cfg->store_path <= CPBUS_STORE_BULK;
+}
+
+int cpbus_create(const cpbus_config* cfg, cpbus_t** out) try {
+  if (!cfg || !out) return CPBUS_EINVAL;
+  *out = nullptr;
+  if (!config_ok(cfg)) return CPBUS_EINVAL;
+  const uint32_t R = cfg->ring_cap ? cfg->ring_cap : 1024;
+  const uint32_t B = cfg->batch_cap ? cfg->batch_cap : std::min(256u, R / 2);
+  const uint32_t K = cfg->timers_per_sub;
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
     snprintf(g_cuda_err, sizeof(g_cuda_err), "no CUDA device visible");
@@ -716,6 +780,13 @@ int cpbus_create(const cpbus_config* cfg, cpbus_t** out) try {
 
 int cpbus_destroy(cpbus_t* b) try {
   if (!b) return CPBUS_EINVAL;
+  if (b->sharded()) {
+    for (size_t k = b->shard_st.size(); k-- > 0;) cpbus_stream_close(b->shard_st[k]);   // attached ends before the owner
+    for (size_t k = b->shards.size(); k-- > 0;) cpbus_destroy(b->shards[k]);
+    if (b->h_batch[0]) cudaFreeHost(b->h_batch[0]);
+    delete b;
+    return CPBUS_OK;
+  }
   cudaSetDevice(b->device);
   if (b->stream) cudaStreamSynchronize(b->stream);
   while (!b->streams.empty()) cpbus_stream_close(b->streams.back());
@@ -808,6 +879,7 @@ int cpbus_source(cpbus_t* b, uint32_t id, char* out, size_t cap, size_t* len) tr
 int cpbus_subscribe_many(cpbus_t* b, const uint32_t* masks, uint32_t n, uint32_t* first_sub_id) try {
   if (!b || !n) return CPBUS_EINVAL;
   if ((uint64_t)b->n_next + n > b->N) return CPBUS_ENOSPC;
+  if (b->sharded()) return sh_subscribe_many(b, masks, n, first_sub_id);
   int rc = dev_guard(b); if (rc) return rc;
   if ((rc = flush_staged(b, b->now))) return rc;   // ordered with publishes (events/bus.go:105-107 takes the same lock)
   const uint32_t first = b->n_next;
@@ -833,6 +905,7 @@ static int push_mask_words(cpbus* b, uint32_t first, uint32_t n);
 int cpbus_subscribe_pairs(cpbus_t* b, uint32_t mask, const cpbus_pair* pairs, uint32_t n_pairs, uint32_t* sub_id) try {
   if (!b || n_pairs > CPBUS_MAX_PAIRS || (n_pairs && !pairs)) return CPBUS_EINVAL;
   for (uint32_t j = 0; j < n_pairs; j++) if (pairs[j].code >= CPBUS_N_CODES) return CPBUS_EINVAL;
+  if (b->sharded()) return sh_subscribe_pairs(b, mask, pairs, n_pairs, sub_id);
   // a pair whose code is already in the mask adds nothing; what is left decides whether a table is needed at all
   uint2 row[CPBUS_MAX_PAIRS];
   uint32_t used = 0;
@@ -868,6 +941,7 @@ int cpbus_subscribe_pairs_many(cpbus_t* b, const uint32_t* masks, const cpbus_pa
     for (uint32_t j = 0; j < n_pairs[i]; j++) if (pairs[(size_t)i * CPBUS_MAX_PAIRS + j].code >= CPBUS_N_CODES) return CPBUS_EINVAL;
   }
   if ((uint64_t)b->n_next + n > b->N) return CPBUS_ENOSPC;
+  if (b->sharded()) return sh_subscribe_pairs_many(b, masks, pairs, n_pairs, n, first_sub_id);
   int rc = dev_guard(b); if (rc) return rc;
   if (!b->d_pairs) {
     if (cudaMalloc((void**)&b->d_pairs, (size_t)b->N * CPBUS_MAX_PAIRS * sizeof(uint2)) != cudaSuccess) {
@@ -902,6 +976,7 @@ int cpbus_subscribe_pairs_many(cpbus_t* b, const uint32_t* masks, const cpbus_pa
 
 int cpbus_unsubscribe(cpbus_t* b, uint32_t sub_id) try {
   if (!b) return CPBUS_EINVAL;
+  if (b->sharded()) return sh_unsubscribe(b, sub_id);
   const uint32_t l = sub_id - b->cfg.sub_id_base;
   if (sub_id < b->cfg.sub_id_base || l >= b->n_next) return CPBUS_ENOENT;
   int rc = dev_guard(b); if (rc) return rc;
@@ -931,6 +1006,7 @@ int cpbus_unsubscribe(cpbus_t* b, uint32_t sub_id) try {
 // NewEventTimer on a channel that was not subscribed, watches/watches.go:37,71) is subscribed to the bus after all.
 int cpbus_set_mask(cpbus_t* b, uint32_t sub_id, uint32_t mask) try {
   if (!b) return CPBUS_EINVAL;
+  if (b->sharded()) return sh_set_mask(b, sub_id, mask);
   const uint32_t l = sub_id - b->cfg.sub_id_base;
   if (sub_id < b->cfg.sub_id_base || l >= b->n_next) return CPBUS_ENOENT;
   if (!b->h_active[l]) return CPBUS_ECLOSED;
@@ -954,6 +1030,7 @@ static int push_mask_words(cpbus* b, uint32_t first, uint32_t n) {
 int cpbus_timer_add(cpbus_t* b, uint32_t sub_id, uint64_t period_ns, uint32_t source_id, int oneshot, uint32_t* timer_id) try {
   if (!b || !period_ns) return CPBUS_EINVAL;
   if (!b->K) return CPBUS_ENOSPC;
+  if (b->sharded()) return sh_timer_add(b, sub_id, period_ns, source_id, oneshot, timer_id);
   const uint32_t l = sub_id - b->cfg.sub_id_base;
   if (sub_id < b->cfg.sub_id_base || l >= b->n_next) return CPBUS_ENOENT;
   int rc = dev_guard(b); if (rc) return rc;
@@ -982,6 +1059,7 @@ int cpbus_timer_add_many(cpbus_t* b, uint32_t first_sub, uint32_t n, uint64_t pe
                          uint32_t source_id0, int oneshot) try {
   if (!b || !period_ns || !n) return CPBUS_EINVAL;
   if (!b->K) return CPBUS_ENOSPC;
+  if (b->sharded()) return sh_timer_add_many(b, first_sub, n, period_ns, source_ids, source_id0, oneshot);
   const uint32_t l0 = first_sub - b->cfg.sub_id_base;
   if (first_sub < b->cfg.sub_id_base || (uint64_t)l0 + n > b->n_next) return CPBUS_ENOENT;
   int rc = dev_guard(b); if (rc) return rc;
@@ -1014,6 +1092,7 @@ int cpbus_timer_add_many(cpbus_t* b, uint32_t first_sub, uint32_t n, uint64_t pe
 
 int cpbus_timer_cancel(cpbus_t* b, uint32_t timer_id) try {
   if (!b) return CPBUS_EINVAL;
+  if (b->sharded()) return sh_timer_cancel(b, timer_id);
   if (!b->K || b->h_timers.empty()) return CPBUS_ENOENT;
   const uint32_t slot_index = timer_id & kTimerSlotMask, gen = timer_id >> kTimerSlotBits;
   const uint32_t l = slot_index / b->K, k = slot_index % b->K;
@@ -1061,6 +1140,7 @@ int cpbus_publish(cpbus_t* b, const cpbus_event* ev, size_t n) try {
 
 int cpbus_send(cpbus_t* b, uint32_t sub_id, const cpbus_event* ev) try {
   if (!b || !ev || ev->code >= CPBUS_N_CODES) return CPBUS_EINVAL;
+  if (b->sharded()) return sh_send(b, sub_id, ev);
   const uint32_t l = sub_id - b->cfg.sub_id_base;
   if (sub_id < b->cfg.sub_id_base || l >= b->n_next) return CPBUS_ENOENT;
   if (!b->h_active[l]) return CPBUS_ECLOSED;   // the mailbox is gone (Go: send on a closed channel panics)
@@ -1094,6 +1174,8 @@ int cpbus_flush(cpbus_t* b) try {
 
 int cpbus_sync(cpbus_t* b) try {
   if (!b) return CPBUS_EINVAL;
+  for (cpbus* s : b->shards) { const int rc = cpbus_sync(s); if (rc) return rc; }
+  if (b->sharded()) return CPBUS_OK;
   int rc = dev_guard(b); if (rc) return rc;
   CK(cudaStreamSynchronize(b->stream));
   return CPBUS_OK;
@@ -1202,6 +1284,7 @@ static int publish_device_impl(cpbus_t* b, const void* d_events, size_t n, uint6
 }
 
 int cpbus_publish_device(cpbus_t* b, const void* d_events, size_t n, uint64_t watermark_ns) try {
+  if (b && b->sharded()) return sh_publish_device(b, d_events, n, watermark_ns);
   return publish_device_impl(b, d_events, n, watermark_ns, false, nullptr, 0);
 } CPBUS_CATCH
 
@@ -1210,12 +1293,13 @@ int cpbus_publish_device(cpbus_t* b, const void* d_events, size_t n, uint64_t wa
 // HBM and publishes it with the batch descriptor; if the caller names the NEXT batch, that one is pulled by the
 // same launch while its stores are in flight, so the following call starts from local memory.  No collective.
 int cpbus_publish_device_staged(cpbus_t* b, const void* d_events, size_t n, uint64_t watermark_ns, const void* d_next, size_t n_next) try {
+  if (b && b->sharded()) return CPBUS_EINVAL;   // the handle already feeds its shards; a peer batch is meant for one shard bus
   return publish_device_impl(b, d_events, n, watermark_ns, true, d_next, n_next);
 } CPBUS_CATCH
 
 // ---- buffers shared between the GPUs of one box (CUDA IPC; NVLink peer mapping on the importing side) ----
 int cpbus_shared_alloc(cpbus_t* b, size_t bytes, void** dptr, unsigned char handle[64]) try {
-  if (!b || !dptr || !handle || !bytes) return CPBUS_EINVAL;
+  if (!b || !dptr || !handle || !bytes || b->sharded()) return CPBUS_EINVAL;
   static_assert(sizeof(cudaIpcMemHandle_t) == 64, "cudaIpcMemHandle_t is 64 bytes");
   int rc = dev_guard(b); if (rc) return rc;
   void* p = nullptr;
@@ -1230,7 +1314,7 @@ int cpbus_shared_alloc(cpbus_t* b, size_t bytes, void** dptr, unsigned char hand
 } CPBUS_CATCH
 
 int cpbus_shared_open(cpbus_t* b, const unsigned char handle[64], void** dptr) try {
-  if (!b || !dptr || !handle) return CPBUS_EINVAL;
+  if (!b || !dptr || !handle || b->sharded()) return CPBUS_EINVAL;
   int rc = dev_guard(b); if (rc) return rc;      // the IMPORTING device must be current: the mapping is made for it
   cudaIpcMemHandle_t h;
   memcpy(&h, handle, 64);
@@ -1242,7 +1326,7 @@ int cpbus_shared_open(cpbus_t* b, const unsigned char handle[64], void** dptr) t
 } CPBUS_CATCH
 
 int cpbus_shared_close(cpbus_t* b, void* dptr) try {
-  if (!b || !dptr) return CPBUS_EINVAL;
+  if (!b || !dptr || b->sharded()) return CPBUS_EINVAL;
   int rc = dev_guard(b); if (rc) return rc;
   CK(cudaStreamSynchronize(b->stream));
   for (int i = 0; i < cpbus::kPrefetch; i++) b->pf_ptr[i] = nullptr;   // prefetched copies of anything in that buffer are void
@@ -1281,9 +1365,16 @@ static int stream_bind(cpbus_stream* st) {
   return CPBUS_OK;
 }
 
+// (a sharded handle uses the stream in lossless mode too: it runs the admission of every shard itself before each put)
+static int stream_create_impl(cpbus* b, uint32_t n_slots, uint32_t n_consumers, cpbus_stream** out, unsigned char handle[64]);
+
 int cpbus_stream_create(cpbus_t* b, uint32_t n_slots, uint32_t n_consumers, cpbus_stream_t** out, unsigned char handle[64]) try {
   if (!b || !out || !handle || n_slots < 4 || n_consumers == 0 || n_consumers > kStreamMaxConsumers) return CPBUS_EINVAL;
-  if (b->lossless) return CPBUS_EINVAL;   // admission would have to see every shard: throughput mode only
+  if (b->lossless || b->sharded()) return CPBUS_EINVAL;   // admission would have to see every shard: throughput mode only
+  return stream_create_impl(b, n_slots, n_consumers, out, handle);
+} CPBUS_CATCH
+
+static int stream_create_impl(cpbus* b, uint32_t n_slots, uint32_t n_consumers, cpbus_stream** out, unsigned char handle[64]) {
   *out = nullptr;
   int rc = dev_guard(b); if (rc) return rc;
   cpbus_stream* st = new (std::nothrow) cpbus_stream();
@@ -1310,11 +1401,11 @@ int cpbus_stream_create(cpbus_t* b, uint32_t n_slots, uint32_t n_consumers, cpbu
   if (cudaMallocHost((void**)&st->h_ack, (size_t)kStreamMaxConsumers * 32) != cudaSuccess) return fail(CPBUS_ENOMEM);
   *out = st;
   return CPBUS_OK;
-} CPBUS_CATCH
+}
 
 int cpbus_stream_open(cpbus_t* b, const unsigned char handle[64], uint32_t consumer_index, cpbus_stream_t** out) try {
   if (!b || !out || !handle || consumer_index == 0 || consumer_index >= kStreamMaxConsumers) return CPBUS_EINVAL;
-  if (b->lossless) return CPBUS_EINVAL;
+  if (b->lossless || b->sharded()) return CPBUS_EINVAL;
   *out = nullptr;
   int rc = dev_guard(b); if (rc) return rc;      // the IMPORTING device must be current: the mapping is made for it
   cpbus_stream* st = new (std::nothrow) cpbus_stream();
@@ -1340,9 +1431,15 @@ int cpbus_stream_open(cpbus_t* b, const unsigned char handle[64], uint32_t consu
 
 // Same-process consumer (one host process driving several GPUs, as a cgo shim would): no IPC handle — the owner's
 // pointer is used directly, with peer access enabled when the consumer's bus lives on another GPU.
+static int stream_attach_impl(cpbus* b, cpbus_stream* owner, uint32_t consumer_index, cpbus_stream** out);
+
 int cpbus_stream_attach(cpbus_t* b, cpbus_stream_t* owner, uint32_t consumer_index, cpbus_stream_t** out) try {
   if (!b || !owner || !owner->owner || !out || consumer_index == 0 || consumer_index >= owner->n_consumers) return CPBUS_EINVAL;
-  if (b->lossless || b->B != owner->B) return CPBUS_EINVAL;
+  if (b->lossless || b->sharded() || b->B != owner->B) return CPBUS_EINVAL;
+  return stream_attach_impl(b, owner, consumer_index, out);
+} CPBUS_CATCH
+
+static int stream_attach_impl(cpbus* b, cpbus_stream* owner, uint32_t consumer_index, cpbus_stream** out) {
   *out = nullptr;
   int rc = dev_guard(b); if (rc) return rc;
   if (b->device != owner->bus->device) {
@@ -1361,7 +1458,7 @@ int cpbus_stream_attach(cpbus_t* b, cpbus_stream_t* owner, uint32_t consumer_ind
   b->streams.push_back(st);
   *out = st;
   return CPBUS_OK;
-} CPBUS_CATCH
+}
 
 int cpbus_stream_close(cpbus_stream_t* st) try {
   if (!st) return CPBUS_EINVAL;
@@ -1455,6 +1552,22 @@ int cpbus_stream_poll(cpbus_stream_t* st, int* ready, size_t* n, uint64_t* now_n
   return CPBUS_OK;
 } CPBUS_CATCH
 
+// One fan-out launch for the next batch of the stream (checks done by the caller).  account = false: the batch's events
+// were already counted where they were published (a sharded handle's cpbus_publish).
+static int stream_launch(cpbus_stream* st, size_t n, uint64_t w, bool account) {
+  cpbus* b = st->bus;
+  const unsigned long long q = st->get_seq + 1;
+  StreamArgs sa;
+  const uint32_t slot = (uint32_t)(q % st->n_slots), slot2 = (uint32_t)((q + 2) % st->n_slots);
+  sa.hdr = &st->hdr[slot]; sa.ack = &st->ack[4 * st->consumer]; sa.seq = q; sa.next_hdr = &st->hdr[slot2];
+  const int rc = launch_fanout(b, st->payload + (size_t)slot * st->B, (uint32_t)n, w, /*staged=*/2,
+                               st->payload + (size_t)slot2 * st->B, b->d_pf_buf + (size_t)((q + 2) % kStreamPrefetch) * b->B, 0,
+                               /*batch_dep=*/false, account, &sa);
+  if (rc) return rc;
+  st->get_seq = q;
+  return CPBUS_OK;
+}
+
 // Every rank (the publisher's included): fan out the next batch of the stream to this GPU's shard.
 int cpbus_stream_fanout(cpbus_stream_t* st, size_t n, uint64_t now_ns) try {
   if (!st || n > st->B) return CPBUS_EINVAL;
@@ -1465,15 +1578,7 @@ int cpbus_stream_fanout(cpbus_stream_t* st, size_t n, uint64_t now_ns) try {
   if (now_ns < b->now) return CPBUS_EORDER;
   if (now_ns - b->last_watermark > max_window(b)) return CPBUS_EORDER;
   b->now = now_ns;
-  const unsigned long long q = st->get_seq + 1;
-  StreamArgs sa;
-  const uint32_t slot = (uint32_t)(q % st->n_slots), slot2 = (uint32_t)((q + 2) % st->n_slots);
-  sa.hdr = &st->hdr[slot]; sa.ack = &st->ack[4 * st->consumer]; sa.seq = q; sa.next_hdr = &st->hdr[slot2];
-  rc = launch_fanout(b, st->payload + (size_t)slot * st->B, (uint32_t)n, now_ns, /*staged=*/2,
-                     st->payload + (size_t)slot2 * st->B, b->d_pf_buf + (size_t)((q + 2) % kStreamPrefetch) * b->B, 0,
-                     /*batch_dep=*/false, /*account=*/true, &sa);
-  if (rc) return rc;
-  st->get_seq = q;
+  if ((rc = stream_launch(st, n, now_ns, /*account=*/true))) return rc;
   b->st.publishes += n; b->seq += n;
   return CPBUS_OK;
 } CPBUS_CATCH
@@ -1501,6 +1606,7 @@ static int copy_slots(cpbus* b, uint32_t l, uint64_t from, size_t n, cpbus_event
 
 int cpbus_drain(cpbus_t* b, uint32_t sub_id, cpbus_event* out, size_t cap, size_t* n, uint64_t* lost) try {
   if (!b || !n || (!out && cap)) return CPBUS_EINVAL;
+  if (b->sharded()) { cpbus* s = sh_owner(b, sub_id); return s ? cpbus_drain(s, sub_id, out, cap, n, lost) : CPBUS_ENOENT; }
   const uint32_t l = sub_id - b->cfg.sub_id_base;
   if (sub_id < b->cfg.sub_id_base || l >= b->n_next) return CPBUS_ENOENT;
   std::lock_guard<std::mutex> g(b->mu);
@@ -1523,6 +1629,7 @@ int cpbus_drain(cpbus_t* b, uint32_t sub_id, cpbus_event* out, size_t cap, size_
 int cpbus_drain_many(cpbus_t* b, uint32_t first_sub, uint32_t n, cpbus_event* out, size_t cap, uint32_t* offsets,
                      uint32_t* counts, size_t* total) try {
   if (!b || !n || !out || !cap || !offsets || !counts || !total || cap > 0xFFFFFFFFull) return CPBUS_EINVAL;
+  if (b->sharded()) return sh_drain_many(b, first_sub, n, out, cap, offsets, counts, total);
   const uint32_t l = first_sub - b->cfg.sub_id_base;
   if (first_sub < b->cfg.sub_id_base || (uint64_t)l + n > b->n_next) return CPBUS_ENOENT;
   std::lock_guard<std::mutex> g(b->mu);
@@ -1555,6 +1662,11 @@ int cpbus_drain_many(cpbus_t* b, uint32_t first_sub, uint32_t n, cpbus_event* ou
 // Device-side consumer: every mailbox of this shard is read to the end and its records are discarded.
 int cpbus_consume_all(cpbus_t* b) try {
   if (!b) return CPBUS_EINVAL;
+  if (b->sharded()) {
+    for (cpbus* s : b->shards) { const int rc = cpbus_consume_all(s); if (rc) return rc; }
+    b->room_lb = b->R;
+    return CPBUS_OK;
+  }
   std::lock_guard<std::mutex> g(b->mu);
   int rc = dev_guard(b); if (rc) return rc;
   if (b->n_next) {
@@ -1569,6 +1681,7 @@ int cpbus_consume_all(cpbus_t* b) try {
 
 int cpbus_peek_window(cpbus_t* b, uint32_t sub_id, cpbus_event* out, size_t cap, size_t* n) try {
   if (!b || !n || (!out && cap)) return CPBUS_EINVAL;
+  if (b->sharded()) { cpbus* s = sh_owner(b, sub_id); return s ? cpbus_peek_window(s, sub_id, out, cap, n) : CPBUS_ENOENT; }
   const uint32_t l = sub_id - b->cfg.sub_id_base;
   if (sub_id < b->cfg.sub_id_base || l >= b->n_next) return CPBUS_ENOENT;
   std::lock_guard<std::mutex> g(b->mu);
@@ -1583,6 +1696,7 @@ int cpbus_peek_window(cpbus_t* b, uint32_t sub_id, cpbus_event* out, size_t cap,
 
 int cpbus_digest(cpbus_t* b, uint32_t first_sub, uint32_t n, cpbus_digest_t* out) try {
   if (!b || !out || !n) return CPBUS_EINVAL;
+  if (b->sharded()) return sh_digest(b, first_sub, n, out);
   const uint32_t l = first_sub - b->cfg.sub_id_base;
   if (first_sub < b->cfg.sub_id_base || (uint64_t)l + n > b->n_next) return CPBUS_ENOENT;
   std::lock_guard<std::mutex> g(b->mu);
@@ -1596,6 +1710,7 @@ int cpbus_digest(cpbus_t* b, uint32_t first_sub, uint32_t n, cpbus_digest_t* out
 
 int cpbus_digest_fold_begin(cpbus_t* b, uint32_t first_sub, uint32_t n, uint32_t* ticket) try {
   if (!b || !ticket || !n) return CPBUS_EINVAL;
+  if (b->sharded()) return sh_digest_fold_begin(b, first_sub, n, ticket);
   const uint32_t l = first_sub - b->cfg.sub_id_base;
   if (first_sub < b->cfg.sub_id_base || (uint64_t)l + n > b->n_next) return CPBUS_ENOENT;
   std::lock_guard<std::mutex> g(b->mu);
@@ -1615,6 +1730,7 @@ int cpbus_digest_fold_begin(cpbus_t* b, uint32_t first_sub, uint32_t n, uint32_t
 
 int cpbus_digest_fold_end(cpbus_t* b, uint32_t ticket, uint64_t out[4]) try {
   if (!b || !out || ticket >= (uint32_t)cpbus::kFoldSlots) return CPBUS_EINVAL;
+  if (b->sharded()) return sh_digest_fold_end(b, ticket, out);
   int rc = dev_guard(b); if (rc) return rc;
   CK(cudaEventSynchronize(b->fold_done[ticket]));
   for (int i = 0; i < 4; i++) out[i] = b->h_fold[4 * ticket + i];
@@ -1631,6 +1747,7 @@ int cpbus_digest_fold(cpbus_t* b, uint32_t first_sub, uint32_t n, uint64_t out[4
 // reading a step's result therefore costs one 256-byte D2H and no extra kernel.
 int cpbus_step_result_begin(cpbus_t* b, uint32_t* ticket) try {
   if (!b || !ticket) return CPBUS_EINVAL;
+  if (b->sharded()) return sh_step_result_begin(b, ticket);
   std::lock_guard<std::mutex> g(b->mu);
   int rc = dev_guard(b); if (rc) return rc;
   const uint32_t t = b->result_next++ % 8;
@@ -1647,6 +1764,7 @@ int cpbus_step_result_begin(cpbus_t* b, uint32_t* ticket) try {
 
 int cpbus_step_result_end(cpbus_t* b, uint32_t ticket, uint64_t out[4]) try {
   if (!b || !out || ticket >= 8) return CPBUS_EINVAL;
+  if (b->sharded()) return sh_step_result_end(b, ticket, out);
   int rc = dev_guard(b); if (rc) return rc;
   CK(cudaEventSynchronize(b->result_done[ticket]));
   out[0] = out[1] = out[2] = out[3] = 0;
@@ -1664,14 +1782,15 @@ static int dbg_resolve(cpbus* b) {
   if (b->dbg_pending.empty()) return CPBUS_OK;
   bool any_marker = false;
   for (const DbgItem& it : b->dbg_pending) any_marker |= it.marker;
+  cpbus* a = b->sharded() ? b->shards[0] : b;   // the bus whose kernel accounted the device batches
   if (any_marker) {
-    int rc = dev_guard(b); if (rc) return rc;
-    CK(cudaMemcpyAsync(b->h_acct->tail, b->d_acct->tail, sizeof(b->h_acct->tail), cudaMemcpyDeviceToHost, b->stream));
-    CK(cudaStreamSynchronize(b->stream));
+    int rc = dev_guard(a); if (rc) return rc;
+    CK(cudaMemcpyAsync(a->h_acct->tail, a->d_acct->tail, sizeof(a->h_acct->tail), cudaMemcpyDeviceToHost, a->stream));
+    CK(cudaStreamSynchronize(a->stream));
   }
   for (const DbgItem& it : b->dbg_pending) {
     if (!it.marker) { dbg_ring_put(b, it.ev); continue; }
-    const DevDbgTail& t = b->h_acct->tail[it.launch % kAcctDbgRing];
+    const DevDbgTail& t = a->h_acct->tail[it.launch % kAcctDbgRing];
     if (t.launch_seq != it.launch) continue;
     for (uint32_t j = 0; j < t.n_kept && j < (uint32_t)kAcctDbgKeep; j++) dbg_ring_put(b, t.ev[j]);
   }
@@ -1698,6 +1817,7 @@ int cpbus_debug_events(cpbus_t* b, cpbus_event* out, size_t cap, size_t* n) try 
 
 int cpbus_stats(cpbus_t* b, cpbus_stats_t* out) try {
   if (!b || !out) return CPBUS_EINVAL;
+  if (b->sharded()) return sh_stats(b, out);
   std::lock_guard<std::mutex> g(b->mu);
   int rc = dev_guard(b); if (rc) return rc;
   CK(cudaMemsetAsync(&b->d_stats->overwritten, 0, sizeof(unsigned long long), b->stream));
@@ -1726,14 +1846,15 @@ int cpbus_stats(cpbus_t* b, cpbus_stats_t* out) try {
 int cpbus_publish_counts(cpbus_t* b, cpbus_pair_count* out, size_t cap, size_t* n) try {
   if (!b || !n || (!out && cap)) return CPBUS_EINVAL;
   std::lock_guard<std::mutex> g(b->mu);
-  int rc = dev_guard(b); if (rc) return rc;
+  cpbus* a = b->sharded() ? b->shards[0] : b;   // the bus whose kernel accounted the device batches
+  int rc = dev_guard(a); if (rc) return rc;
   std::unordered_map<uint64_t, uint64_t> merged;
   for (size_t i = 0; i < b->pub_pairs.keys.size(); i++) if (b->pub_pairs.keys[i]) merged[b->pub_pairs.keys[i] - 1] += b->pub_pairs.cnts[i];
-  if (b->launch_seq) {
+  if (a->launch_seq) {
     std::vector<unsigned long long> keys(kAcctPairSlots), cnts(kAcctPairSlots);
-    CK(cudaMemcpyAsync(keys.data(), b->d_acct->pair_key, sizeof(unsigned long long) * kAcctPairSlots, cudaMemcpyDeviceToHost, b->stream));
-    CK(cudaMemcpyAsync(cnts.data(), b->d_acct->pair_cnt, sizeof(unsigned long long) * kAcctPairSlots, cudaMemcpyDeviceToHost, b->stream));
-    CK(cudaStreamSynchronize(b->stream));
+    CK(cudaMemcpyAsync(keys.data(), a->d_acct->pair_key, sizeof(unsigned long long) * kAcctPairSlots, cudaMemcpyDeviceToHost, a->stream));
+    CK(cudaMemcpyAsync(cnts.data(), a->d_acct->pair_cnt, sizeof(unsigned long long) * kAcctPairSlots, cudaMemcpyDeviceToHost, a->stream));
+    CK(cudaStreamSynchronize(a->stream));
     for (uint32_t i = 0; i < kAcctPairSlots; i++) if (keys[i]) merged[keys[i] - 1] += cnts[i];
   }
   std::vector<std::pair<uint64_t, uint64_t>> v(merged.begin(), merged.end());
@@ -1744,10 +1865,460 @@ int cpbus_publish_counts(cpbus_t* b, cpbus_pair_count* out, size_t cap, size_t* 
 } CPBUS_CATCH
 
 int cpbus_device_ptrs(cpbus_t* b, void** ring, void** ctl) try {
-  if (!b) return CPBUS_EINVAL;
+  if (!b || b->sharded()) return CPBUS_EINVAL;   // the layout is per shard
   if (ring) *ring = b->d_ring;
   if (ctl) *ctl = b->d_ctl;
   return CPBUS_OK;
 } CPBUS_CATCH
 
+
+// ---- one handle over several GPUs (include/cpbus.h: cpbus_create_sharded) ----
+int cpbus_shard_range(uint32_t n_max_subs, uint32_t n_shards, uint32_t shard, uint32_t* first, uint32_t* count) {
+  if (!n_shards || shard >= n_shards || !first || !count) return CPBUS_EINVAL;
+  const uint32_t base = n_max_subs / n_shards, extra = n_max_subs % n_shards;
+  *first = shard * base + std::min(shard, extra);
+  *count = base + (shard < extra ? 1u : 0u);
+  return CPBUS_OK;
+}
+
+int cpbus_create_sharded(const cpbus_config* cfg, const int32_t* devices, uint32_t n_shards, cpbus_t** out) try {
+  if (!cfg || !out) return CPBUS_EINVAL;
+  *out = nullptr;
+  if (!devices || !n_shards || n_shards > kStreamMaxConsumers || cfg->stream || !config_ok(cfg) || cfg->n_max_subs < n_shards)
+    return CPBUS_EINVAL;
+  cpbus_config c = *cfg;
+  if (n_shards == 1) { c.device = devices[0]; return cpbus_create(&c, out); }
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+    snprintf(g_cuda_err, sizeof(g_cuda_err), "no CUDA device visible");
+    return CPBUS_ENODEV;
+  }
+  for (uint32_t k = 0; k < n_shards; k++) if (devices[k] < 0 || devices[k] >= ndev) return CPBUS_EINVAL;
+  cpbus* h = new (std::nothrow) cpbus();
+  if (!h) return CPBUS_ENOMEM;
+  auto fail = [&](int code) { cpbus_destroy(h); return code; };
+  h->R = cfg->ring_cap ? cfg->ring_cap : 1024;
+  h->B = cfg->batch_cap ? cfg->batch_cap : std::min(256u, h->R / 2);
+  h->cfg = *cfg; h->cfg.ring_cap = h->R; h->cfg.batch_cap = h->B; h->cfg.device = devices[0];
+  h->N = cfg->n_max_subs; h->K = cfg->timers_per_sub; h->device = devices[0];
+  h->lossless = cfg->flags & CPBUS_CFG_LOSSLESS; h->use_digest = cfg->flags & CPBUS_CFG_DIGEST;
+  h->room_lb = h->R;
+  for (uint32_t k = 0; k < n_shards; k++) {
+    uint32_t first = 0, count = 0;
+    cpbus_shard_range(cfg->n_max_subs, n_shards, k, &first, &count);
+    c = *cfg; c.n_max_subs = count; c.sub_id_base = cfg->sub_id_base + first; c.device = devices[k];
+    cpbus* s = nullptr;
+    const int rc = cpbus_create(&c, &s);
+    if (rc) return fail(rc);
+    h->shards.push_back(s); h->shard_first.push_back(first);
+  }
+  // the handle's stream: shard 0 owns it, the others attach in-process (peer access when they live on another GPU).  16 slots
+  // let the host run that many flushes ahead of the slowest shard before cpbus_stream_put waits for it.
+  unsigned char ipc[64];
+  cpbus_stream* st0 = nullptr;
+  int rc = stream_create_impl(h->shards[0], 16, n_shards, &st0, ipc);
+  if (rc) return fail(rc);
+  h->shard_st.push_back(st0);
+  for (uint32_t k = 1; k < n_shards; k++) {
+    cpbus_stream* st = nullptr;
+    if ((rc = stream_attach_impl(h->shards[k], st0, k, &st))) return fail(rc);
+    h->shard_st.push_back(st);
+  }
+  // staging: pinned, portable and mapped, so that the admission kernel of every shard can read it in place
+  if ((rc = dev_guard(h))) return fail(rc);
+  if (cudaHostAlloc((void**)&h->h_batch[0], (size_t)h->B * sizeof(cpbus_event), cudaHostAllocPortable | cudaHostAllocMapped) != cudaSuccess)
+    return fail(CPBUS_ENOMEM);
+  if (cudaHostGetDevicePointer((void**)&h->d_batch_host, h->h_batch[0], 0) != cudaSuccess) return fail(CPBUS_ECUDA);
+  h->intern.emplace(std::string(), 0u);
+  h->sources.emplace_back();
+  *out = h;
+  return CPBUS_OK;
+} CPBUS_CATCH
+
 }  // extern "C"
+
+namespace {
+
+uint32_t sh_index(const cpbus* h, uint32_t l) {   // shard holding local id l < N
+  return (uint32_t)(std::upper_bound(h->shard_first.begin(), h->shard_first.end(), l) - h->shard_first.begin()) - 1u;
+}
+uint32_t sh_end(const cpbus* h, uint32_t k) { return k + 1 < h->shards.size() ? h->shard_first[k + 1] : h->N; }
+
+cpbus* sh_owner(const cpbus* h, uint32_t sub_id) {
+  const uint32_t l = sub_id - h->cfg.sub_id_base;
+  if (sub_id < h->cfg.sub_id_base || l >= h->n_next) return nullptr;
+  return h->shards[sh_index(h, l)];
+}
+
+// f(shard index, first local id, count) for each shard's piece of local ids [l, l + n), in id order; stops at an error
+template <class F>
+int sh_pieces(const cpbus* h, uint32_t l, uint32_t n, F f) {
+  const uint64_t hi = (uint64_t)l + n;
+  for (uint32_t lo = l; lo < hi;) {
+    const uint32_t k = sh_index(h, lo), e = (uint32_t)std::min<uint64_t>(hi, sh_end(h, k));
+    const int rc = f(k, lo, e - lo);
+    if (rc) return rc;
+    lo = e;
+  }
+  return CPBUS_OK;
+}
+
+bool sh_in_range(const cpbus* h, uint32_t first_sub, uint32_t n) {
+  return first_sub >= h->cfg.sub_id_base && (uint64_t)(first_sub - h->cfg.sub_id_base) + n <= h->n_next;
+}
+
+// The shards follow the handle's clock: a shard's timers are armed relative to its `now`, and its own flush (which every
+// membership / timer call runs first) then finds nothing to do.
+void sh_sync_clocks(cpbus* h) {
+  for (cpbus* s : h->shards) { s->now = h->now; s->last_watermark = h->last_watermark; }
+}
+
+void sh_retire_oneshots(cpbus* h) {   // where one bus would retire its fired one-shots: on every shard at once
+  for (cpbus* s : h->shards) retire_oneshots(s, s->last_watermark);
+  if (timers_armed(h) == 0) h->min_period = UINT64_MAX;
+}
+
+// Lossless admission over every shard: the handle keeps one room bound like a single bus; when it is used up, the admission
+// kernel runs on every shard (each reads the pinned staging buffer in place) and the results merge as if one kernel had seen
+// every mailbox: any overflow refuses, the shortest prefix wins, the fullest mailbox sets the new bound.
+int sh_admit(cpbus* h, uint32_t n, uint64_t w, bool* ok, uint32_t* prefix) {
+  *ok = true; *prefix = n;
+  if (h->n_next == 0) return CPBUS_OK;
+  const uint64_t need = admit_need(n, h->K, timers_armed(h) > 0, h->min_period, h->last_watermark, w);
+  if (h->room_lb >= need) { h->room_lb -= need; h->st.admit_skipped++; return CPBUS_OK; }
+  int rc;
+  for (cpbus* s : h->shards)
+    if (s->n_next && ((rc = dev_guard(s)) || (rc = admit_launch(s, h->d_batch_host, n, w)))) return rc;
+  unsigned long long overflow = 0, deficit = 0, used = 0;
+  for (cpbus* s : h->shards) {
+    if (!s->n_next) continue;
+    if ((rc = dev_guard(s))) return rc;
+    CK(cudaStreamSynchronize(s->stream));
+    overflow += s->h_stats->admit_overflow;
+    deficit = std::max(deficit, s->h_stats->admit_deficit);
+    used = std::max(used, s->h_stats->admit_max_used);
+  }
+  h->st.admit_passes++;
+  *ok = overflow == 0;
+  if (!*ok) *prefix = n - (uint32_t)std::min<unsigned long long>(n, deficit);
+  h->room_lb = used >= h->R ? 0 : h->R - used;
+  return CPBUS_OK;
+}
+
+// One flush of a handle = one put of the staged records into the stream + one stream fan-out per shard (flush_staged's rules).
+int flush_sharded(cpbus* h, uint64_t w) {
+  const uint32_t n = (uint32_t)h->n_staged;
+  const uint32_t timers = timers_armed(h);
+  if ((n == 0 && timers == 0) || (n == 0 && w == h->last_watermark)) {
+    if (n == 0 && timers == 0) h->last_watermark = std::max(h->last_watermark, w);
+    sh_sync_clocks(h);
+    return CPBUS_OK;
+  }
+  if (h->n_next == 0) {   // no mailbox yet: one bus launches nothing and drops the batch, so does the handle
+    h->n_staged = 0;
+    sh_sync_clocks(h);
+    return CPBUS_OK;
+  }
+  bool ok = true;
+  uint32_t m = n;
+  int rc;
+  if (h->lossless && (rc = sh_admit(h, n, w, &ok, &m))) return rc;
+  if (!ok) {
+    if (m == 0) return CPBUS_EAGAIN;
+    w = h->h_batch[0][m - 1].ts_ns;   // the prefix every mailbox of every shard can take, with the ticks due by its last event
+  }
+  for (cpbus* s : h->shards) if (*(volatile unsigned int*)s->h_err) return CPBUS_ETIMEDOUT;
+  // the default put waits (bounded) for the slot's previous batch: its fan-outs are already queued behind earlier puts
+  if ((rc = cpbus_stream_put(h->shard_st[0], h->h_batch[0], m, w, CPBUS_PUT_RAW))) return rc;
+  for (size_t k = 0; k < h->shards.size(); k++) {
+    if ((rc = dev_guard(h->shards[k]))) return rc;
+    if ((rc = stream_launch(h->shard_st[k], m, w, /*account=*/false))) return rc;
+  }
+  h->last_watermark = w;
+  sh_sync_clocks(h);
+  if (!ok) {
+    memmove(h->h_batch[0], h->h_batch[0] + m, (size_t)(n - m) * sizeof(cpbus_event));   // (the put copied the prefix out)
+    h->n_staged = n - m;
+    h->room_lb = 0;
+    h->st.admit_partial++;
+    return CPBUS_EAGAIN;
+  }
+  h->n_staged = 0;
+  return CPBUS_OK;
+}
+
+// flush the handle (membership and timer calls are ordered with publishes, events/bus.go:105-122), then work on the shards
+int sh_prepare(cpbus* h) {
+  int rc = dev_guard(h); if (rc) return rc;
+  return flush_staged(h, h->now);
+}
+
+int sh_subscribe_many(cpbus* h, const uint32_t* masks, uint32_t n, uint32_t* first_sub_id) {
+  int rc = sh_prepare(h); if (rc) return rc;
+  const uint32_t first = h->n_next;
+  rc = sh_pieces(h, first, n, [&](uint32_t k, uint32_t lo, uint32_t cnt) {
+    const int r = cpbus_subscribe_many(h->shards[k], masks ? masks + (lo - first) : nullptr, cnt, nullptr);
+    if (!r) h->n_next += cnt;
+    return r;
+  });
+  if (rc) return rc;
+  if (first_sub_id) *first_sub_id = h->cfg.sub_id_base + first;
+  return CPBUS_OK;
+}
+
+int sh_subscribe_pairs(cpbus* h, uint32_t mask, const cpbus_pair* pairs, uint32_t n_pairs, uint32_t* sub_id) {
+  if (h->n_next >= h->N) return CPBUS_ENOSPC;
+  int rc = sh_prepare(h); if (rc) return rc;
+  if ((rc = cpbus_subscribe_pairs(h->shards[sh_index(h, h->n_next)], mask, pairs, n_pairs, sub_id))) return rc;
+  h->n_next++;
+  return CPBUS_OK;
+}
+
+int sh_subscribe_pairs_many(cpbus* h, const uint32_t* masks, const cpbus_pair* pairs, const uint32_t* n_pairs, uint32_t n,
+                            uint32_t* first_sub_id) {
+  int rc = sh_prepare(h); if (rc) return rc;
+  const uint32_t first = h->n_next;
+  rc = sh_pieces(h, first, n, [&](uint32_t k, uint32_t lo, uint32_t cnt) {
+    const size_t i = lo - first;
+    const int r = cpbus_subscribe_pairs_many(h->shards[k], masks + i, pairs + i * CPBUS_MAX_PAIRS, n_pairs + i, cnt, nullptr);
+    if (!r) h->n_next += cnt;
+    return r;
+  });
+  if (rc) return rc;
+  if (first_sub_id) *first_sub_id = h->cfg.sub_id_base + first;
+  return CPBUS_OK;
+}
+
+int sh_unsubscribe(cpbus* h, uint32_t sub_id) {
+  cpbus* s = sh_owner(h, sub_id);
+  if (!s) return CPBUS_ENOENT;
+  int rc = sh_prepare(h); if (rc) return rc;
+  return cpbus_unsubscribe(s, sub_id);
+}
+
+int sh_set_mask(cpbus* h, uint32_t sub_id, uint32_t mask) {
+  cpbus* s = sh_owner(h, sub_id);
+  if (!s) return CPBUS_ENOENT;
+  if (!s->h_active[sub_id - s->cfg.sub_id_base]) return CPBUS_ECLOSED;
+  int rc = sh_prepare(h); if (rc) return rc;
+  return cpbus_set_mask(s, sub_id, mask);
+}
+
+// timer ids of a handle are global slots: (id - sub_id_base) * K + k, with the shard's generation bits
+int sh_timer_add(cpbus* h, uint32_t sub_id, uint64_t period_ns, uint32_t source_id, int oneshot, uint32_t* timer_id) {
+  cpbus* s = sh_owner(h, sub_id);
+  if (!s) return CPBUS_ENOENT;
+  int rc = sh_prepare(h); if (rc) return rc;
+  sh_retire_oneshots(h);
+  h->any_timer = true;
+  uint32_t local = 0;
+  if ((rc = cpbus_timer_add(s, sub_id, period_ns, source_id, oneshot, &local))) return rc;
+  if (!oneshot) h->min_period = std::min(h->min_period, period_ns);
+  const uint32_t shift = (s->cfg.sub_id_base - h->cfg.sub_id_base) * h->K;
+  if (timer_id) *timer_id = ((local & kTimerSlotMask) + shift) | (local & ~kTimerSlotMask);
+  return CPBUS_OK;
+}
+
+int sh_timer_add_many(cpbus* h, uint32_t first_sub, uint32_t n, uint64_t period_ns, const uint32_t* source_ids, uint32_t source_id0,
+                      int oneshot) {
+  if (!sh_in_range(h, first_sub, n)) return CPBUS_ENOENT;
+  int rc = sh_prepare(h); if (rc) return rc;
+  sh_retire_oneshots(h);
+  h->any_timer = true;
+  const uint32_t l0 = first_sub - h->cfg.sub_id_base;
+  // all or nothing, as on one bus: check every piece before arming any
+  rc = sh_pieces(h, l0, n, [&](uint32_t k, uint32_t lo, uint32_t cnt) {
+    const cpbus* s = h->shards[k];
+    for (uint32_t i = lo - h->shard_first[k], e = i + cnt; i < e; i++) {
+      if (!s->h_active[i]) return (int)CPBUS_ECLOSED;
+      if (!s->h_timers.empty() && s->h_timers[(size_t)i * s->K].active) return (int)CPBUS_ENOSPC;
+    }
+    return (int)CPBUS_OK;
+  });
+  if (rc) return rc;
+  if ((rc = sh_pieces(h, l0, n, [&](uint32_t k, uint32_t lo, uint32_t cnt) {
+        const uint32_t i = lo - l0;
+        return cpbus_timer_add_many(h->shards[k], h->cfg.sub_id_base + lo, cnt, period_ns, source_ids ? source_ids + i : nullptr,
+                                    source_id0 + i, oneshot);
+      })))
+    return rc;
+  if (!oneshot) h->min_period = std::min(h->min_period, period_ns);
+  return CPBUS_OK;
+}
+
+int sh_timer_cancel(cpbus* h, uint32_t timer_id) {
+  if (!h->K || !h->any_timer) return CPBUS_ENOENT;
+  const uint32_t slot = timer_id & kTimerSlotMask, l = slot / h->K;
+  if (l >= h->n_next) return CPBUS_ENOENT;
+  int rc = sh_prepare(h); if (rc) return rc;
+  sh_retire_oneshots(h);
+  const uint32_t k = sh_index(h, l);
+  rc = cpbus_timer_cancel(h->shards[k], (slot - h->shard_first[k] * h->K) | (timer_id & ~kTimerSlotMask));
+  if (timers_armed(h) == 0) h->min_period = UINT64_MAX;
+  return rc;
+}
+
+int sh_send(cpbus* h, uint32_t sub_id, const cpbus_event* ev) {
+  cpbus* s = sh_owner(h, sub_id);
+  if (!s) return CPBUS_ENOENT;
+  if (!s->h_active[sub_id - s->cfg.sub_id_base]) return CPBUS_ECLOSED;
+  int rc = dev_guard(h); if (rc) return rc;
+  if ((rc = stage_one(h, ev->code, ev->source_id, sub_id, CPBUS_F_UNICAST))) return rc;   // global target: the owner's kernel takes it
+  h->st.publishes++;
+  return CPBUS_OK;
+}
+
+// one slice that every shard's launch can take: shard 0 reads the batch locally, the others pull it from shard 0's GPU
+int sh_device_slice(cpbus* h, const cpbus_event* d_events, size_t n, uint64_t w) {
+  for (size_t k = 0; k < h->shards.size(); k++) {
+    const int rc = publish_device_impl(h->shards[k], d_events, n, w, /*staged=*/k > 0, nullptr, 0);
+    if (rc) return rc;
+  }
+  cpbus* s0 = h->shards[0];
+  for (const DbgItem& it : s0->dbg_pending) {   // shard 0's kernel accounted the batch: its debug-ring markers move to the handle
+    h->dbg_pending.push_back(it);
+    if (h->dbg_pending.size() > (size_t)kAcctDbgRing) h->dbg_pending.pop_front();
+  }
+  for (cpbus* s : h->shards) s->dbg_pending.clear();
+  h->now = h->last_watermark = w;
+  h->st.publishes += n; h->seq += n;
+  sh_sync_clocks(h);
+  return CPBUS_OK;
+}
+
+int sh_publish_device(cpbus* h, const void* d_events, size_t n, uint64_t watermark_ns) {
+  if ((!d_events && n) || ((uintptr_t)d_events & 31u)) return CPBUS_EINVAL;
+  if (h->lossless) return CPBUS_EINVAL;   // admission would have to read the batch from every shard: not supported
+  int rc = dev_guard(h); if (rc) return rc;
+  if ((rc = flush_staged(h, h->now))) return rc;
+  if (watermark_ns < h->now) return CPBUS_EORDER;
+  const cpbus_event* ev = (const cpbus_event*)d_events;
+  const uint64_t window = max_window(h);
+  if (n <= h->B && watermark_ns - h->last_watermark <= window) return sh_device_slice(h, ev, n, watermark_ns);
+  // the same cut as publish_device_split, planned once for all shards
+  std::vector<uint64_t> ts(n), wm;
+  std::vector<size_t> end;
+  cpbus* s0 = h->shards[0];
+  if (n) {
+    CK(cudaMemcpy2DAsync(ts.data(), 8, reinterpret_cast<const unsigned char*>(ev) + offsetof(cpbus_event, ts_ns), sizeof(cpbus_event),
+                         8, n, cudaMemcpyDeviceToHost, s0->stream));
+    CK(cudaStreamSynchronize(s0->stream));
+  }
+  if ((rc = split_plan(ts.data(), n, h->B, h->now, watermark_ns, window, end, wm))) return rc;
+  size_t i = 0;
+  for (size_t k = 0; k < end.size(); k++) {
+    if ((rc = sh_device_slice(h, ev + i, end[k] - i, wm[k]))) return rc;
+    h->st.device_splits++;
+    i = end[k];
+  }
+  return CPBUS_OK;
+}
+
+int sh_drain_many(cpbus* h, uint32_t first_sub, uint32_t n, cpbus_event* out, size_t cap, uint32_t* offsets, uint32_t* counts,
+                  size_t* total) {
+  if (!sh_in_range(h, first_sub, n)) return CPBUS_ENOENT;
+  const uint32_t l0 = first_sub - h->cfg.sub_id_base;
+  size_t used = 0, tot = 0;
+  const int rc = sh_pieces(h, l0, n, [&](uint32_t k, uint32_t lo, uint32_t cnt) {
+    uint32_t* offs = offsets + (lo - l0);
+    uint32_t* cnts = counts + (lo - l0);
+    if (used >= cap) {   // no room left: these mailboxes stay untouched for the next call
+      memset(offs, 0, cnt * sizeof(uint32_t)); memset(cnts, 0, cnt * sizeof(uint32_t));
+      return (int)CPBUS_OK;
+    }
+    size_t t = 0, hi = 0;
+    const int r = cpbus_drain_many(h->shards[k], h->cfg.sub_id_base + lo, cnt, out + used, cap - used, offs, cnts, &t);
+    if (r) return r;
+    for (uint32_t i = 0; i < cnt; i++)
+      if (cnts[i]) { hi = std::max<size_t>(hi, (size_t)offs[i] + cnts[i]); offs[i] += (uint32_t)used; }
+    used += hi; tot += t;
+    return (int)CPBUS_OK;
+  });
+  if (rc) return rc;
+  *total = tot;
+  return CPBUS_OK;
+}
+
+int sh_digest(cpbus* h, uint32_t first_sub, uint32_t n, cpbus_digest_t* out) {
+  if (!sh_in_range(h, first_sub, n)) return CPBUS_ENOENT;
+  const uint32_t l0 = first_sub - h->cfg.sub_id_base;
+  return sh_pieces(h, l0, n, [&](uint32_t k, uint32_t lo, uint32_t cnt) {
+    return cpbus_digest(h->shards[k], h->cfg.sub_id_base + lo, cnt, out + (lo - l0));
+  });
+}
+
+int sh_digest_fold_begin(cpbus* h, uint32_t first_sub, uint32_t n, uint32_t* ticket) {
+  if (!sh_in_range(h, first_sub, n)) return CPBUS_ENOENT;
+  const uint32_t slot = h->fold_next++ % cpbus::kFoldSlots;
+  auto& parts = h->fold_parts[slot];
+  parts.clear();
+  const int rc = sh_pieces(h, first_sub - h->cfg.sub_id_base, n, [&](uint32_t k, uint32_t lo, uint32_t cnt) {
+    uint32_t t = 0;
+    const int r = cpbus_digest_fold_begin(h->shards[k], h->cfg.sub_id_base + lo, cnt, &t);
+    if (!r) parts.emplace_back(k, t);
+    return r;
+  });
+  if (rc) return rc;
+  *ticket = slot;
+  return CPBUS_OK;
+}
+
+int sh_digest_fold_end(cpbus* h, uint32_t ticket, uint64_t out[4]) {
+  out[0] = out[1] = out[2] = out[3] = 0;
+  for (const auto& p : h->fold_parts[ticket]) {   // the fold's own combination: sums, XOR, sum of n
+    uint64_t o[4];
+    const int rc = cpbus_digest_fold_end(h->shards[p.first], p.second, o);
+    if (rc) return rc;
+    out[0] += o[0]; out[1] += o[1]; out[2] ^= o[2]; out[3] += o[3];
+  }
+  return CPBUS_OK;
+}
+
+int sh_step_result_begin(cpbus* h, uint32_t* ticket) {
+  const uint32_t t = h->result_next++ % 8;
+  auto& parts = h->result_parts[t];
+  parts.clear();
+  for (cpbus* s : h->shards) {
+    uint32_t st = 0;
+    const int rc = cpbus_step_result_begin(s, &st);
+    if (rc) return rc;
+    parts.push_back(st);
+  }
+  *ticket = t;
+  return CPBUS_OK;
+}
+
+// deliveries, ticks and digest sums add up over the shards; the launch ordinal is the same on every shard (shard 0's)
+int sh_step_result_end(cpbus* h, uint32_t ticket, uint64_t out[4]) {
+  out[0] = out[1] = out[2] = out[3] = 0;
+  const auto& parts = h->result_parts[ticket];
+  for (size_t k = 0; k < parts.size(); k++) {
+    uint64_t o[4];
+    const int rc = cpbus_step_result_end(h->shards[k], parts[k], o);
+    if (rc) return rc;
+    out[0] += o[0]; out[1] += o[1]; out[2] += o[2];
+    if (k == 0) out[3] = o[3];
+  }
+  return CPBUS_OK;
+}
+
+int sh_stats(cpbus* h, cpbus_stats_t* out) {
+  *out = h->st;
+  out->deliveries = out->ticks = out->batches = out->kernel_launches = out->overwritten = 0;
+  out->n_subs = out->n_timers = 0;
+  for (size_t k = 0; k < h->shards.size(); k++) {
+    cpbus_stats_t s{};
+    const int rc = cpbus_stats(h->shards[k], &s);
+    if (rc) return rc;
+    out->deliveries += s.deliveries; out->ticks += s.ticks; out->batches += s.batches; out->kernel_launches += s.kernel_launches;
+    out->overwritten += s.overwritten; out->n_subs += s.n_subs; out->n_timers += s.n_timers;
+    if (k == 0) for (int c = 0; c < CPBUS_N_CODES; c++) out->published_by_code[c] += s.published_by_code[c];   // device batches (shard 0's kernel)
+  }
+  if (timers_armed(h) == 0) h->min_period = UINT64_MAX;   // (the shards' statistics retired their fired one-shots)
+  out->now_ns = h->now;
+  out->intern_entries = h->sources.size(); out->intern_bytes = h->intern_bytes;
+  out->ephemeral_live = h->eph_live; out->ephemeral_recycled = h->eph_recycled;
+  return CPBUS_OK;
+}
+
+}  // namespace

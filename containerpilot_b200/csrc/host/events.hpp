@@ -189,13 +189,18 @@ class EventBus {   // events/bus.go:12-22
   enum class Clock { Virtual, Monotonic };
   // NewEventBus() — events/bus.go:72-88.  Clock::Virtual: time moves only through Advance() (tests);
   // Clock::Monotonic: a pump thread feeds std::chrono::steady_clock every millisecond.
-  explicit EventBus(Clock clock = Clock::Monotonic, uint32_t n_max_subs = 256, uint32_t mailbox_cap = 1024) : clock_(clock) {
+  // `devices` non-empty: the subscribers are sharded over these GPUs behind one handle (cpbus_create_sharded); nothing
+  // else about the bus changes.
+  explicit EventBus(Clock clock = Clock::Monotonic, uint32_t n_max_subs = 256, uint32_t mailbox_cap = 1024,
+                    std::vector<int> devices = {}) : clock_(clock) {
     cpbus_config cfg{};
     cfg.n_max_subs = n_max_subs; cfg.ring_cap = mailbox_cap; cfg.batch_cap = mailbox_cap >= 512 ? 256 : mailbox_cap / 2;
     cfg.timers_per_sub = 4; cfg.flags = CPBUS_CFG_LOSSLESS | CPBUS_CFG_DIGEST; cfg.device = -1;
     batch_cap_ = cfg.batch_cap;
-    int rc = cpbus_create(&cfg, &h_);
-    if (rc) throw std::runtime_error(std::string("cpbus_create: ") + cpbus_strerror(rc) + " " + cpbus_last_cuda_error());
+    const std::vector<int32_t> devs(devices.begin(), devices.end());
+    int rc = devs.empty() ? cpbus_create(&cfg, &h_) : cpbus_create_sharded(&cfg, devs.data(), (uint32_t)devs.size(), &h_);
+    if (rc) throw std::runtime_error(std::string(devs.empty() ? "cpbus_create: " : "cpbus_create_sharded: ") + cpbus_strerror(rc) +
+                                     " " + cpbus_last_cuda_error());
     start_ = std::chrono::steady_clock::now();
     life_->h = h_;
     { std::lock_guard<std::mutex> g(CurrentMutex()); CurrentSlot() = this; }

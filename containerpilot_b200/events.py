@@ -115,7 +115,10 @@ class Chan:
 
 
 class EventBus:
-    """EventBus — events/bus.go:12-22.  NewEventBus() == EventBus()."""
+    """EventBus — events/bus.go:12-22.  NewEventBus() == EventBus().
+
+    `EventBus(devices=[0, 1, ...])` puts the subscribers on several GPUs behind one handle (`Bus(devices=...)`); nothing
+    else about the API changes."""
 
     def __init__(self, n_max_subs: int = 64, ring_cap: int = 1024, batch_cap: int = 256, timers_per_sub: int = 4,
                  lossless: bool = True, **kw):

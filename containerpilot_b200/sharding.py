@@ -13,6 +13,8 @@ Two drivers over the same C-ABI:
 """
 from __future__ import annotations
 
+import ctypes as C
+
 import numpy as np
 
 from . import _native as nat
@@ -20,12 +22,13 @@ from .bus import Bus, EVENT_DTYPE
 
 
 def shard_range(n_total: int, world: int, rank: int) -> tuple[int, int]:
-    """Contiguous, near-even partition: returns (first_global_id, count) of `rank`'s shard."""
+    """Contiguous, near-even partition: returns (first_global_id, count) of `rank`'s shard (libcpbus `cpbus_shard_range`, the
+    partition `cpbus_create_sharded` uses)."""
     if not (0 <= rank < world):
         raise ValueError("rank out of range")
-    base, extra = divmod(n_total, world)
-    first = rank * base + min(rank, extra)
-    return first, base + (1 if rank < extra else 0)
+    first, count = C.c_uint32(), C.c_uint32()
+    nat.check(nat.load().cpbus_shard_range(n_total, world, rank, C.byref(first), C.byref(count)), "cpbus_shard_range")
+    return first.value, count.value
 
 
 def owner_of(sub_id: int, n_total: int, world: int) -> int:

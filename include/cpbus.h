@@ -145,6 +145,36 @@ typedef struct cpbus cpbus_t;
 int cpbus_create(const cpbus_config* cfg, cpbus_t** out);
 int cpbus_destroy(cpbus_t* bus);
 
+/* ---- one handle over several GPUs ----------------------------------------------------------------------------------------
+ * G shard buses behind ONE handle: every other cpbus_* entry point takes it unchanged, and every value a caller reads back
+ * equals what one bus created with the same cfg returns (status codes, records, lost, digests, folds, step results, debug
+ * events, publish counts, source ids, statistics) — except cpbus_stats.batches and .kernel_launches, which are sums over
+ * the shards.  cfg means what it means for cpbus_create (total capacity, ring, batch, timers, flags, store path, grid);
+ * cfg->device is ignored: shard k lives on devices[k] (a device may repeat).  n_shards == 1 is exactly cpbus_create on
+ * devices[0].  CPBUS_EINVAL (before any device is touched): what cpbus_create rejects, devices == NULL, n_shards == 0 or
+ * > 64, n_max_subs < n_shards, cfg->stream != NULL.  If a shard cannot be created, what was made is destroyed.
+ *   Ids.  Shard k owns the contiguous global ids sub_id_base + cpbus_shard_range(n_max_subs, n_shards, k); ids are handed
+ *   out in order from sub_id_base as on one bus, so a fleet that fills the handle spreads evenly and a few subscribers all
+ *   sit on shard 0.  Timer ids are global slots ((id - sub_id_base) * K + k, with the generation bits).
+ *   Routing.  Intern/source: one table at the handle.  Ranges (subscribe_many, subscribe_pairs_many, timer_add_many, digest,
+ *   digest_fold*, drain_many) are cut at the shard boundaries; drain_many keeps its contract when cap is short (every run is
+ *   complete and FIFO, a mailbox left out has counts[i] = 0).  Single-subscriber calls go to the owner shard after the
+ *   staged events are flushed.  cpbus_step_result_end: deliveries, ticks and digest sums added over the shards, the launch
+ *   ordinal of shard 0.
+ *   Data path.  The handle stages events like one bus (seq = publish ordinal, ts = its clock).  A flush puts the staged
+ *   records into a stream owned by shard 0 and launches one stream fan-out per shard (cpbus_stream_*: each shard's lead CTA
+ *   pulls the batch); cpbus_advance cuts clock steps at the narrowest timer window over the shards.  Lossless mode: a flush
+ *   delivers, on every shard, the longest prefix every mailbox of every shard can take (the admission pass runs on each shard
+ *   when the handle's room bound is used up) and returns CPBUS_EAGAIN for the rest, as one bus does.
+ *   cpbus_publish_device: throughput mode only (shard 0 reads the batch locally, the others pull it from shard 0's GPU;
+ *   oversize batches are cut once for all shards; shard 0's kernel accounts them); CPBUS_EINVAL in lossless mode.
+ *   CPBUS_EINVAL on a handle: cpbus_publish_device_staged, cpbus_stream_create/open/attach, cpbus_shared_*, cpbus_device_ptrs. */
+int cpbus_create_sharded(const cpbus_config* cfg, const int32_t* devices, uint32_t n_shards, cpbus_t** out);
+/* The id partition of cpbus_create_sharded, host-only (no device): shard `shard` of n_shards holds local ids
+ * [*first, *first + *count) of n_max_subs; the first n_max_subs % n_shards shards hold one more.  CPBUS_EINVAL: n_shards == 0,
+ * shard >= n_shards, or a NULL output. */
+int cpbus_shard_range(uint32_t n_max_subs, uint32_t n_shards, uint32_t shard, uint32_t* first, uint32_t* count);
+
 /* ---- Event.Source interning (events/events.go:12; SURVEY F7) ---- */
 int cpbus_intern(cpbus_t* bus, const char* s, size_t len, uint32_t* source_id);
 /* copies at most cap bytes; *len receives the full length.  CPBUS_ENOENT: unknown id, or an ephemeral id whose
